@@ -5,6 +5,10 @@
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 \
            --master-port P bench.py --gpus N --steps K --warmup W       # our arm, N GPUs (weak scaling)
     python bench.py --impl reference --gpus 1 --steps K --warmup W      # reference CPU path on host cores
+    python bench.py --gpus 1 --steps K --warmup W --dump-outputs DIR    # + the last timed step's outputs as .npy
+
+The inputs are seeded: the same arguments give the same inputs on every run, so the dumped outputs
+of two builds can be compared element for element.
 
 A step = one pass of the hot path (log-softmax statistics -> alpha/beta lattice -> dense gradient)
 over one batch of synthetic logits; workload = BASELINE config "N=128, T=150, L=20, A=5000 fp32"
@@ -305,6 +309,34 @@ def time_steps(torch, fn, steps, warmup=3, flush=None):
         e1.synchronize()
         tot += e0.elapsed_time(e1)
     return tot / steps
+
+
+DUMP_SAMPLE = 1 << 20
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(torch, out_dir, costs, grads, labels_np, loss):
+    """Writes what the timed path handed its caller in the last timed step, as float32 .npy files:
+    the per-utterance costs, the step's summed loss, and the gradient (8 GB at the flagship shape) at
+    fixed seeded positions: DUMP_SAMPLE elements anywhere, DUMP_SAMPLE cells' blank entries and
+    DUMP_SAMPLE cells' entries at the cell's next label.  The gradient samples have a fixed size, so
+    every workload's dump stays below DUMP_LIMIT_BYTES."""
+    N, T, U, V = grads.shape
+    rng = np.random.default_rng(0)
+    anywhere = rng.integers(0, grads.numel(), size=DUMP_SAMPLE)
+    blank = rng.integers(0, N * T * U, size=DUMP_SAMPLE) * V
+    cell = rng.integers(0, N * T * (U - 1), size=DUMP_SAMPLE)        # (n, t, u) with u < U - 1
+    n, t, u = cell // (T * (U - 1)), cell // (U - 1) % T, cell % (U - 1)
+    label = ((n * T + t) * U + u) * V + labels_np[n, u]
+    flat = grads.view(-1)
+    out = {"costs": costs, "loss": loss}
+    for name, idx in (("grads_sample", anywhere), ("grads_blank", blank), ("grads_label", label)):
+        out[name] = flat[torch.as_tensor(idx, device=grads.device)]
+    out = {name: t.float().cpu().numpy() for name, t in out.items()}
+    assert sum(a.nbytes for a in out.values()) <= DUMP_LIMIT_BYTES
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def oracle_check_utterance(torch, acts_b, labels_b, T_b, L_b, cost_b, grads_b):
@@ -622,6 +654,9 @@ def run_b200_arm(args):
         del flush
     launches = wr.last_launch_count() * args.steps
     wr.set_profiling(False)
+    if args.dump_outputs and rank == 0:
+        # before the legs below reuse costs / grads
+        dump_outputs(torch, args.dump_outputs, costs, grads, labels_np, loss2[(state["k"] - 1) & 1])
 
     # ---- secondary, reported separately (SURVEY 8(d)): ragged lengths ~U[0.5,1]*max, seed 2.
     # Padded cells are not read (pass 1 skips them, pass 2 writes zeros), so bytes move less.
@@ -826,7 +861,13 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-c5", action="store_true", help="skip the config-5 strong-scaling leg")
     ap.add_argument("--quick", action="store_true", help="skip the reference-GPU and other-workload legs")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write rank 0's outputs of the last timed step to DIR/<name>.npy (b200 arm)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs applies to the b200 arm")
     if args.impl == "reference":
         run_reference_arm(args)
     else:
@@ -839,7 +880,8 @@ def main():
                    "--master-port", os.environ.get("MASTER_PORT", "29517"), os.path.abspath(__file__),
                    "--gpus", str(args.gpus), "--steps", str(args.steps), "--warmup", str(args.warmup),
                    "--workload", args.workload] + (["--no-cpu-baseline"] if args.no_cpu_baseline else []) + \
-                  (["--no-c5"] if args.no_c5 else []) + (["--quick"] if args.quick else [])
+                  (["--no-c5"] if args.no_c5 else []) + (["--quick"] if args.quick else []) + \
+                  (["--dump-outputs", os.path.abspath(args.dump_outputs)] if args.dump_outputs else [])
             raise SystemExit(subprocess.call(cmd))
         run_b200_arm(args)
 

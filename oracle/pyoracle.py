@@ -180,11 +180,15 @@ def log_softmax_np(x):
     return (x - m) - np.log(np.exp(x - m).sum(axis=-1, keepdims=True))
 
 
+def logits_grad(lp, g):
+    """log_softmax backward: gradient wrt the logits from the gradient g wrt the log-probs lp."""
+    return g - np.exp(lp) * g.sum(axis=-1, keepdims=True)
+
+
 def ref_cpu_logits(acts, labels, act_lens, label_lens, blank=0, threads=0):
     """logits -> log_softmax -> reference CPU lib -> log_softmax backward (what warprnnt_pytorch
     composes on CPU, pytorch_binding/warprnnt_pytorch/__init__.py:95-98 + autograd)."""
     acts = np.ascontiguousarray(acts)
     lp = log_softmax_np(acts)
     costs, g = ref_cpu_logprobs(lp, labels, act_lens, label_lens, blank, True, threads)
-    dx = g - np.exp(lp) * g.sum(axis=-1, keepdims=True)
-    return costs, dx.astype(acts.dtype)
+    return costs, logits_grad(lp, g).astype(acts.dtype)

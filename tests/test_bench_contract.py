@@ -31,6 +31,38 @@ def test_reference_arm_other_ranks_exit_quietly():
     assert out.returncode == 0 and out.stdout.strip() == ""
 
 
+def test_argument_rejections():
+    for extra in (["--steps", "0"], ["--impl", "reference", "--dump-outputs", "out"]):
+        out = subprocess.run([sys.executable, BENCH] + extra, capture_output=True, text=True, timeout=120)
+        assert out.returncode == 2 and "error:" in out.stderr, (extra, out.stderr[-500:])
+
+
+def test_dump_outputs_files(tmp_path):
+    """dump_outputs on small CPU tensors: float32 files, the sampled entries are the gradient's."""
+    import numpy as np
+    import torch
+    sys.path.insert(0, ROOT)
+    import bench
+    N, T, U, V = 3, 5, 4, 7
+    grads = torch.randn(N, T, U, V)
+    labels = np.random.default_rng(0).integers(1, V, size=(N, U - 1)).astype(np.int32)
+    costs = torch.randn(N)
+    bench.dump_outputs(torch, str(tmp_path), costs, grads, labels, costs.sum().reshape(1))
+    out = {p.stem: np.load(p) for p in tmp_path.iterdir()}
+    assert sorted(out) == ["costs", "grads_blank", "grads_label", "grads_sample", "loss"]
+    assert all(a.dtype == np.float32 for a in out.values())
+    assert sum(a.nbytes for a in out.values()) <= bench.DUMP_LIMIT_BYTES
+    assert np.array_equal(out["costs"], costs.numpy()) and np.isclose(out["loss"][0], costs.sum().item())
+    g = grads.numpy()
+    assert np.isin(out["grads_blank"], g[..., 0]).all()
+    at_labels = np.take_along_axis(g[:, :, :U - 1], labels[:, None, :, None].astype(np.int64), 3)
+    assert np.isin(out["grads_label"], at_labels).all()
+    assert np.isin(out["grads_sample"], g).all()
+    again = tmp_path / "again"
+    bench.dump_outputs(torch, str(again), costs, grads, labels, costs.sum().reshape(1))
+    assert all(np.array_equal(np.load(again / (k + ".npy")), v) for k, v in out.items())
+
+
 def test_b200_arm_has_no_cpu_fallback():
     import torch
     if torch.cuda.is_available():

@@ -3,10 +3,12 @@
   1. the reference test-suite's own known-answer vectors (tests/golden/known_answers.json)
   2. outputs of the reference itself on seeded random cases (tests/golden/ref_cases.npz,
      produced by the compiled reference CPU library + the reference numpy model)
-  3. live agreement with oracle/_ref/libwarprnnt_ref_cpu.so where that file exists
+  3. outputs of the compiled reference CPU library (oracle/_ref/libwarprnnt_ref_cpu.so) on
+     seeded inputs, stored in tests/golden/ref_live_cases.npz
 """
+import os
+
 import numpy as np
-import pytest
 
 from oracle import pyoracle
 
@@ -68,30 +70,43 @@ def test_against_committed_reference_outputs(ref_cases):
             assert not g32[b, T:].any() and not g32[b, :, U:].any(), name
 
 
-@pytest.mark.skipif(not pyoracle.have_ref_cpu(), reason="oracle/_ref not built")
-def test_live_against_compiled_reference():
+LIVE_SHAPES = [(3, 11, 6, 10), (2, 50, 10, 15), (65, 10, 5, 5), (1, 50, 15, 20)]
+REF_LIVE = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "ref_live_cases.npz")
+
+
+def live_cases():
+    """Seeded inputs of test_live_against_compiled_reference, one (acts, labels, tl, ul) per shape."""
     rng = np.random.default_rng(7)
-    for (N, T, U, V) in [(3, 11, 6, 10), (2, 50, 10, 15), (65, 10, 5, 5), (1, 50, 15, 20)]:
+    for (N, T, U, V) in LIVE_SHAPES:
         acts = rng.random((N, T, U, V), dtype=np.float32)      # U[0,1) like tests/random.cpp:13-20
         labels = rng.integers(1, V, size=(N, U - 1)).astype(np.int32)
         tl = rng.integers(T // 2 + 1, T + 1, size=N).astype(np.int32)
         ul = rng.integers(0, U, size=N).astype(np.int32)
         tl[0], ul[0] = T, U - 1
+        yield acts, labels, tl, ul
+
+
+def test_live_against_compiled_reference():
+    """The compiled reference CPU library's outputs on live_cases() are stored in
+    tests/golden/ref_live_cases.npz (tests/golden/make_golden_ref_runs.py cpu)."""
+    with np.load(REF_LIVE) as z:
+        stored = dict(z)
+    for k, (acts, labels, tl, ul) in enumerate(live_cases()):
+        ref = {name: stored["%d.%s" % (k, name)] for name in
+               ("costs_f32", "grads_f32", "costs_fwd_f32", "costs_f64", "grads_f64")}
         lp = pyoracle.log_softmax_np(acts)
-        c_ref, g_ref = pyoracle.ref_cpu_logprobs(lp, labels, tl, ul, 0, threads=2)
         c_orc, g_orc = pyoracle.rnnt_logprobs(lp, labels, tl, ul, 0, threads=2)
-        assert np.allclose(c_orc, c_ref, rtol=1e-6, atol=1e-5)
+        assert np.allclose(c_orc, ref["costs_f32"], rtol=1e-6, atol=1e-5)
         # fp32 noise floor: exp(lp+alpha+beta-ll) with |ll|~100 has ~4 ulp(100)=3e-5 abs error in
         # BOTH implementations (each is 3e-5 from the fp64 result); the fp64 comparison below is tight
-        assert np.allclose(g_orc, g_ref, rtol=1e-4, atol=5e-5)
+        assert np.allclose(g_orc, ref["grads_f32"], rtol=1e-4, atol=5e-5)
         # forward-only entry (gradients == NULL -> score_forward, rnnt_entrypoint.cpp:70-72)
-        c_fwd, _ = pyoracle.ref_cpu_logprobs(lp, labels, tl, ul, 0, want_grad=False)
         c_of, _ = pyoracle.rnnt_logprobs(lp, labels, tl, ul, 0, want_grad=False)
-        assert np.allclose(c_of, c_fwd, rtol=1e-6, atol=1e-5)
+        assert np.allclose(c_of, ref["costs_fwd_f32"], rtol=1e-6, atol=1e-5)
         # logits convention = reference CPU lib composed with log-softmax fwd/bwd
-        c2, dx_ref = pyoracle.ref_cpu_logits(acts.astype(np.float64), labels, tl, ul, 0)
+        dx_ref = pyoracle.logits_grad(pyoracle.log_softmax_np(acts.astype(np.float64)), ref["grads_f64"])
         c3, dx_orc, _ = pyoracle.rnnt_logits(acts.astype(np.float64), labels, tl, ul, 0)
-        assert np.allclose(c3, c2, rtol=1e-12)
+        assert np.allclose(c3, ref["costs_f64"], rtol=1e-12)
         assert np.allclose(dx_orc, dx_ref, rtol=1e-9, atol=1e-13)
 
 

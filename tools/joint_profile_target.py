@@ -1,6 +1,6 @@
 import os, sys
 import numpy as np, torch
-ROOT = "/root/repo"
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, os.path.join(ROOT, "warp-transducer_b200"))
 from warprnnt_pytorch.joint import AddJointRNNTLoss
 dev = torch.device("cuda:0")
